@@ -10,6 +10,8 @@ random-init weights, synthetic inputs, labels=None, logits for all positions.  A
 global batch; with N ranks the global batch is split by sample (strong scaling, no collective on the data path).
 
 One JSON line is printed by rank 0 (see the field list in DESIGN.md §Measurement).
+
+  python bench.py ... --dump-outputs DIR   # also write what the last timed step computed as DIR/<name>.npy (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -24,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from untouched (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -173,7 +176,7 @@ def cpu_threads() -> int:
     return max(1, min(usable_cores(), physical_cores_one_socket()))
 
 
-def cpu_reference_sample(cfgs, hyper, L, steps, warmup, seed=1234, state_dict=None, inputs=None, budget_s=240.0):
+def cpu_reference_sample(cfgs, hyper, L, steps, warmup, seed=1234, state_dict=None, inputs=None):
     """Time the reference's own CPU implementation of the path on a bounded sample of the workload: ONE sample (B=1)
     image+audio+text, full model depth, fp32.
 
@@ -223,7 +226,6 @@ def cpu_reference_sample(cfgs, hyper, L, steps, warmup, seed=1234, state_dict=No
             return o["logits"], o["embeds"]
         what = "oracle/macaw_oracle.py (port; oracle/_ref absent)"
     times, T, out = [], None, None
-    t_begin = time.perf_counter()
     for i in range(warmup + steps):
         t0 = time.perf_counter()
         out = run()
@@ -231,9 +233,6 @@ def cpu_reference_sample(cfgs, hyper, L, steps, warmup, seed=1234, state_dict=No
         T = out[0].shape[1]
         if i >= warmup:
             times.append(dt)
-        # keep the whole arm within the budget: stop early once at least one timed step exists
-        if (time.perf_counter() - t_begin) + dt > budget_s and times:
-            break
     sec = sum(times) / len(times)
     return dict(value=T / sec, unit=UNIT, cores=cores, kind=kind, steps_timed=len(times), sec_per_step=sec,
                 logits=out[0], embeds=out[1],
@@ -398,7 +397,7 @@ def run_decode(args, cfgs, hyper, rank, local_rank, world):
     for _ in range(max(1, min(args.warmup, 2))):
         run(n_new)
     t1 = min(run(1)[0] for _ in range(2))           # prefill + first token
-    tn = min(run(n_new)[0] for _ in range(max(1, min(args.steps, 3))))
+    tn = min(run(n_new)[0] for _ in range(args.steps))
     ms_step = (tn - t1) / (n_new - 1)
     hbm, _, _, src = load_peaks()
     wbytes = sum(p.numel() * p.element_size() for n_, p in model.named_parameters() if n_.startswith("llm.model.layers") or n_ == "llm.lm_head.weight")
@@ -411,6 +410,29 @@ def run_decode(args, cfgs, hyper, rank, local_rank, world):
             "prefill_ms": t1, "ms_per_decode_step": ms_step,
             "roofline": {"bound": "hbm", "achieved": wbytes / (ms_step / 1e3) / 1e9, "peak": hbm, "unit": "GB/s",
                          "frac": floor_ms / ms_step, "peak_source": src, "algorithmic_bytes_per_step": wbytes}}), flush=True)
+
+
+# ---------------------------------------------------------------------------------------------------- output dump
+DUMP_SAMPLE_BYTES = 48 * 2 ** 20  # logits_sample.npy
+DUMP_LAST_BYTES = 16 * 2 ** 20    # logits_last.npy: 64 MiB in all
+
+
+def dump_outputs(logits, out_dir: str) -> None:
+    """Write the (B, T, V) logits of one prefill step as float32 .npy files under `out_dir`:
+      logits_last.npy    (b, V)  next-token logits of the first b = min(B, 16 MiB / (4 V)) samples (all 32 at cfg4);
+      logits_sample.npy  (n, V)  n = min(B T, 48 MiB / (4 V)) rows of the (B T, V) logits, flattened batch-major, at the
+                                 positions of a seed-0 torch.randperm, sorted (the same rows for the same arguments)."""
+    import numpy as np
+
+    B, T, V = logits.shape
+    flat = logits.reshape(B * T, V)
+    n = min(B * T, DUMP_SAMPLE_BYTES // (4 * V))
+    rows = torch.randperm(B * T, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    arrays = {"logits_last": logits[: min(B, DUMP_LAST_BYTES // (4 * V)), -1, :],
+              "logits_sample": flat[rows.to(flat.device)]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------- main
@@ -437,7 +459,14 @@ def main():
     ap.add_argument("--dtype", default=DEFAULT_DTYPE, choices=["bf16", "fp16"],
                     help="storage / tensor-core operand format of the prefill arm (fp32 accumulation either way); the "
                          "reference itself runs fp16 (train.sh --fp16 True)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="prefill: after the timed steps, write what the last one computed (rank 0's logits, float32, a "
+                         "fixed seeded sample) as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "prefill"):
+        ap.error("--dump-outputs applies to the prefill benchmark of the b200 implementation")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -463,9 +492,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 5))
         warm = min(args.warmup, 1)
-        cb = cpu_reference_sample(cfgs, hyper, L, steps, warm)
+        cb = cpu_reference_sample(cfgs, hyper, L, args.steps, warm)
         line = {
             "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": cb["steps_timed"], "warmup": warm, "ms_per_step": cb["sec_per_step"] * 1e3,
@@ -573,6 +601,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     value = B_global * T * args.steps / (ms_max / 1e3)
+    if args.dump_outputs and rank == 0:  # here: the next region overwrites the CUDA graph's output buffers
+        dump_outputs(logits, args.dump_outputs)
 
     # ---- timed region 2: end to end through the public call with HOST (pinned) buffers: H2D of every input + forward
     #      + D2H of the step's result (next-token logits of every sample)
@@ -641,8 +671,7 @@ def main():
                                                                for k, v in one.items()})
             g_log = model({k: (v.to(dev) if isinstance(v, torch.Tensor) else v) for k, v in one.items()}).logits
         g_emb, g_log = g_emb.float().cpu(), g_log.float().cpu()
-        cb = cpu_reference_sample(cfgs, hyper, L, steps=1, warmup=0, state_dict=model.state_dict(), inputs=one,
-                                  budget_s=120.0)
+        cb = cpu_reference_sample(cfgs, hyper, L, steps=1, warmup=0, state_dict=model.state_dict(), inputs=one)
         cpu = {"value": cb["value"], "unit": UNIT, "cores": cb["cores"], "kind": cb["kind"], "sample": cb["sample"]}
         r_log, r_emb = cb["logits"].float(), cb["embeds"].float()
         n_prefix = r_emb.shape[1] - L

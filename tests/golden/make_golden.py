@@ -145,6 +145,29 @@ def main():
     assert torch.equal(pe_ref, pe_orc), float((pe_ref - pe_orc).abs().max())
     np.savez_compressed(os.path.join(HERE, "video_pe_40x24.npz"), pe=pe_ref.numpy())
     print("[golden] video positional encoding: bit-exact vs reference loop")
+    reference_outputs(modeling)
+
+
+def reference_outputs(modeling):
+    """What the reference itself returns, recorded for the tests that compare with it:
+    ref_image_audio.npz   fp32 `MM_LLMs.forward` of the tiny model on an image+audio batch (tests/test_oracle.py);
+    ref_state_dict_resized.json   names / shapes / dtypes of the state_dict the reference writes after
+                                  `model.llm.resize_token_embeddings(V + 7)` (run_clm_llms.py:495; tests/test_wire.py)."""
+    _, model, _, _ = build_reference(modeling, gen.TINY)
+    B, L, seed, pad = 2, 11, 7, 2
+    mods = ("image", "audio")
+    inp = gen.make_inputs(gen.TINY, B, L, seed=seed, modalities=mods, pad_tail=pad)
+    with torch.no_grad():
+        out = model(inp)
+    np.savez_compressed(os.path.join(HERE, "ref_image_audio.npz"), B=B, L=L, seed=seed, pad_tail=pad,
+                        modalities=np.array(list(mods), dtype="U8"), logits=out.logits.float().numpy(),
+                        loss=float(out.loss))
+    print(f"[golden] reference image+audio forward: logits {tuple(out.logits.shape)}, loss {float(out.loss):.6f}")
+    model.llm.resize_token_embeddings(gen.TINY["llama"]["vocab_size"] + 7)
+    layout = {k: [list(v.shape), str(v.dtype).replace("torch.", "")] for k, v in model.state_dict().items()}
+    with open(os.path.join(HERE, "ref_state_dict_resized.json"), "w") as f:
+        json.dump(layout, f, indent=0, sort_keys=True)
+    print(f"[golden] reference state_dict after resize_token_embeddings: {len(layout)} entries")
 
 
 if __name__ == "__main__":

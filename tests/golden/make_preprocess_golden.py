@@ -55,6 +55,14 @@ def whisper_log_mel(audio: torch.Tensor) -> torch.Tensor:
     return (log_spec + 4.0) / 4.0
 
 
+def mel_frames(i: int) -> np.ndarray:
+    """Frames of clip i stored in the fixture: every frame of the padded clip (its silent tail compresses to nothing), a
+    seeded sample of 400 of the trimmed clip's 3000 frames (audio everywhere: stored whole it would be ~0.8 MB)."""
+    if i == 0:
+        return np.arange(3000)
+    return np.sort(np.random.default_rng(i).choice(3000, 400, replace=False))
+
+
 def main():
     tf, Image = reference_transform()
     out = {}
@@ -77,7 +85,8 @@ def main():
         a = torch.from_numpy(gen.synth_audio(secs, seed=i))
         lm = whisper_log_mel(a)
         assert lm.shape == (80, 3000)
-        out[f"mel{i}"] = lm.numpy().astype(np.float32)
+        out[f"mel{i}_cols"] = mel_frames(i)
+        out[f"mel{i}"] = lm.numpy().astype(np.float32)[:, out[f"mel{i}_cols"]]
     np.savez_compressed(os.path.join(HERE, "preprocess.npz"), **out)
     print({k: v.shape for k, v in out.items()}, os.path.getsize(os.path.join(HERE, "preprocess.npz")) // 1024, "KiB")
 

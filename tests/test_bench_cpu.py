@@ -40,6 +40,29 @@ def test_b200_arm_refuses_to_run_without_cuda():
     assert r.returncode != 0 and "no CPU fallback" in (r.stderr + r.stdout)
 
 
+def test_dump_outputs_is_float32_bounded_and_repeatable(tmp_path):
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    B, T, V = 3, 50, 1000
+    logits = torch.randn(B, T, V, generator=torch.Generator().manual_seed(3)).to(torch.float16)
+    for d in ("a", "b"):
+        bench.dump_outputs(logits, str(tmp_path / d))
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["logits_last.npy", "logits_sample.npy"]
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "logits_last.npy"), logits[:, -1].float().numpy())
+    # every row fits the budget here, so the sorted sample is the whole flattened output in order
+    assert np.array_equal(np.load(tmp_path / "a" / "logits_sample.npy"), logits.float().reshape(B * T, V).numpy())
+    # at the benchmark's shape the two files stay within 64 MiB
+    rows = min(32 * 528, bench.DUMP_SAMPLE_BYTES // (4 * 32000)) + min(32, bench.DUMP_LAST_BYTES // (4 * 32000))
+    assert rows * 32000 * 4 <= 64 * 2 ** 20
+
+
 def test_synth_inputs_and_cores():
     sys.path.insert(0, ROOT)
     import bench

@@ -1,5 +1,4 @@
-"""CPU tier: the oracle (oracle/macaw_oracle.py) against the golden vectors minted from the unmodified reference, and
-— when /root/reference exists (build container) — against the live reference in-process."""
+"""CPU tier: the oracle (oracle/macaw_oracle.py) against the golden vectors minted from the unmodified reference."""
 import os
 
 import numpy as np
@@ -155,16 +154,14 @@ def test_philox_known_answers():
     assert abs(float((m != 0).mean()) - 0.9) < 0.03
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree only exists in the build container")
-def test_oracle_vs_live_reference():
-    from tests.golden import make_golden as MG
-
-    modeling = MG.import_reference()
-    cfg, model, shapes, weights = MG.build_reference(modeling, gen.TINY)
-    hp = O.hp_from_config(cfg)
-    inp = gen.make_inputs(gen.TINY, 2, 11, seed=7, modalities=("image", "audio"), pad_tail=2)
-    with torch.no_grad():
-        out = model(inp)
-    o = O.forward(inp, {k: v for k, v in model.state_dict().items()}, hp)
-    assert H.rel_err(o["logits"], out.logits) < 1e-4
-    assert abs(float(o["loss"]) - float(out.loss)) < 1e-4
+def test_oracle_vs_live_reference(tiny_weights):
+    """fp32 oracle vs the reference's own fp32 forward of the tiny model on an image+audio batch with labels
+    (tests/golden/ref_image_audio.npz, recorded from the unmodified reference by make_golden.reference_outputs)."""
+    spec, hp, weights = tiny_weights
+    z = np.load(os.path.join(H.GOLDEN, "ref_image_audio.npz"))
+    inp = gen.make_inputs(spec, int(z["B"]), int(z["L"]), seed=int(z["seed"]),
+                          modalities=tuple(str(m) for m in z["modalities"]), pad_tail=int(z["pad_tail"]))
+    o = O.forward(inp, weights, hp)
+    assert tuple(o["logits"].shape) == z["logits"].shape
+    assert H.rel_err(o["logits"], torch.from_numpy(z["logits"])) < 1e-4
+    assert abs(float(o["loss"]) - float(z["loss"])) < 1e-4
