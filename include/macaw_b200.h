@@ -385,6 +385,40 @@ int32_t mm_colsum(const void* x, int64_t ldx, int32_t rows, int32_t cols, float*
 int32_t mm_adamw(void* p, const void* g, float* master, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                  float eps, float weight_decay, int32_t step, const int32_t* step_dev, float grad_scale, void* stream);
 
+/* Device-resident optimizer state of the scheduled update (one per optimizer; every step-dependent scalar lives here, so
+ * a CUDA graph of the step replays with the right values).  Written by mm_grad_norm, read by mm_adamw_sched.
+ * Initialise with step = skipped = arrived = 0, clip_coef = 1, finite = 1, apply = 0. */
+typedef struct mm_opt_state {
+  int32_t step;      /* optimizer steps taken (skipped steps not counted): the bias-correction step of the update */
+  int32_t skipped;   /* steps skipped because their gradients were not finite */
+  float lr;          /* learning rate of the latest step: base_lr * lambda(step - 1) */
+  float clip_coef;   /* gradient multiplier of the latest step: min(1, max_norm / (grad_norm + 1e-6)), 1 without clipping */
+  float grad_norm;   /* global L2 norm of the latest step's gradients, before clipping (0 when no pass ran) */
+  int32_t finite;    /* 1 when every gradient element of the latest step was finite */
+  int32_t apply;     /* 1 when the latest step updates the parameters (0: skipped) */
+  int32_t arrived;   /* CTA arrival counter of mm_grad_norm; 0 between launches */
+} mm_opt_state;
+/* Learning-rate schedules of transformers.optimization (lambda of the 0-based step; num_cycles = 0.5 for cosine). */
+#define MM_SCHED_CONSTANT 0
+#define MM_SCHED_CONSTANT_WITH_WARMUP 1
+#define MM_SCHED_LINEAR 2
+#define MM_SCHED_COSINE 3
+/* Partial sums of mm_grad_norm: `partials` holds MM_GRAD_NORM_PARTS doubles. */
+#define MM_GRAD_NORM_PARTS 1024
+/* Global gradient norm + step bookkeeping of the scheduled update.  table: device int64 [n_tensors][2] = (address, numel)
+ * of the bf16 gradients to include.  The sum of squares is deterministic (fixed partition: fp32 per thread over runs of at
+ * most 64 elements, fp64 across threads and CTAs, summed in a fixed order): bit-identical run to run and rank to rank.
+ * The last CTA writes grad_norm, finite, clip_coef (max_norm <= 0: no clipping); then, if the gradients are finite or
+ * skip_nonfinite == 0, step += 1, lr = base_lr * lambda(step - 1) (fp64), apply = 1; otherwise skipped += 1, apply = 0.
+ * n_tensors == 0 runs the scalar work only (a schedule without clipping or the finiteness check). */
+int32_t mm_grad_norm(const int64_t* table, int32_t n_tensors, double* partials, mm_opt_state* state, float max_norm,
+                     int32_t skip_nonfinite, float base_lr, int32_t schedule, int32_t warmup_steps, int32_t total_steps,
+                     void* stream);
+/* mm_adamw with lr, the gradient multiplier (clip_coef) and the bias-correction step read from *state; a step with
+ * state->apply == 0 leaves p, master, m and v untouched. */
+int32_t mm_adamw_sched(void* p, const void* g, float* master, float* m, float* v, int64_t n, float beta1, float beta2,
+                       float eps, float weight_decay, const mm_opt_state* state, void* stream);
+
 /* Backward of the absorbed alignment attention through its (V + 2)-key softmax (reference: autograd of
  * nn.MultiheadAttention, modeling.py:986-987 / 1007-1008 / 1025-1026).  See train_kernels.cu for the formulas. */
 int32_t mm_align_softmax_bwd(const float* G, int64_t ldg, const void* P_unnorm_f16, int64_t ldp, const float* inv_l,

@@ -137,6 +137,8 @@ SIGNATURES = {
     "mm_embed_scatter_add": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_i32, c_i32, c_vp, c_vp]),
     "mm_colsum": (c_i32, [c_vp, c_i64, c_i32, c_i32, c_vp, c_vp]),
     "mm_adamw": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_f32, c_f32, c_i32, c_vp, c_f32, c_vp]),
+    "mm_grad_norm": (c_i32, [c_vp, c_i32, c_vp, c_vp, c_f32, c_i32, c_f32, c_i32, c_i32, c_i32, c_vp]),
+    "mm_adamw_sched": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_f32, c_f32, c_f32, c_f32, c_vp, c_vp]),
     "mm_image_preprocess": (c_i32, [C.POINTER(ImageArgs), c_vp]),
     "mm_log_mel": (c_i32, [c_vp, c_i32, c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_vp]),
     "mm_align_softmax_bwd": (c_i32, [c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_f32, c_vp, c_vp, c_i64, c_vp, c_i32,

@@ -470,10 +470,20 @@ __global__ void colsum_kernel(const bf16* __restrict__ x, long long ldx, int row
 //   m = b1 m + (1-b1) g;  v = b2 v + (1-b2) g^2;  w -= lr (m/bc1 / (sqrt(v/bc2) + eps) + wd w);  p = bf16(w)
 // 8 elements per thread and iteration: one 128-bit gradient load, two 128-bit loads / stores per fp32 state tensor, one
 // 128-bit parameter store (28 bytes of HBM traffic per parameter; the scalar kernel below reached 4.5 TB/s of it).
+// kSched (mm_adamw_sched): lr, the gradient multiplier and the step come from the device optimizer state, and a skipped
+// step returns before touching memory.
+template <bool kSched>
 __global__ void __launch_bounds__(256) adamw_vec8_kernel(bf16* __restrict__ p, const bf16* __restrict__ g, float* __restrict__ w,
                                                          float* __restrict__ m, float* __restrict__ v, long long n8, float lr,
                                                          float b1, float b2, float eps, float wd, float inv_bc1, float inv_bc2,
-                                                         float gscale, const int* __restrict__ step_dev) {
+                                                         float gscale, const int* __restrict__ step_dev,
+                                                         const mm_opt_state* __restrict__ st) {
+  if constexpr (kSched) {
+    if (!st->apply) return;
+    lr = st->lr;
+    gscale = st->clip_coef;
+    step_dev = &st->step;
+  }
   if (step_dev != nullptr) {
     const float t = static_cast<float>(*step_dev);
     inv_bc1 = 1.f / (1.f - powf(b1, t));
@@ -508,9 +518,17 @@ __global__ void __launch_bounds__(256) adamw_vec8_kernel(bf16* __restrict__ p, c
   }
 }
 
+template <bool kSched>
 __global__ void adamw_kernel(bf16* __restrict__ p, const bf16* __restrict__ g, float* __restrict__ w, float* __restrict__ m,
                              float* __restrict__ v, long long n, float lr, float b1, float b2, float eps, float wd,
-                             float inv_bc1, float inv_bc2, float gscale, const int* __restrict__ step_dev) {
+                             float inv_bc1, float inv_bc2, float gscale, const int* __restrict__ step_dev,
+                             const mm_opt_state* __restrict__ st) {
+  if constexpr (kSched) {
+    if (!st->apply) return;
+    lr = st->lr;
+    gscale = st->clip_coef;
+    step_dev = &st->step;
+  }
   if (step_dev != nullptr) {  // step count read on the device: the launch can be replayed from a CUDA graph
     const float t = static_cast<float>(*step_dev);
     inv_bc1 = 1.f / (1.f - powf(b1, t));
@@ -527,6 +545,119 @@ __global__ void adamw_kernel(bf16* __restrict__ p, const bf16* __restrict__ g, f
     v[i] = vi;
     w[i] = wi;
     p[i] = __float2bfloat16(wi);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------ global gradient norm
+// Sum of squares over a table of bf16 gradient tensors, then the optimizer's per-step scalars (clip coefficient, step,
+// learning rate).  Work unit: a chunk of kNormChunk consecutive elements of one tensor; the chunks of all tensors are
+// numbered in table order and chunk c belongs to CTA c % gridDim.x.  Each thread squares its kNormVecs 8-element runs of
+// a chunk in fp32 and adds that run sum to its fp64 accumulator; CTA sums (fixed shuffle tree) go to partials[blockIdx.x]
+// and the last CTA to arrive adds them in index order.  Nothing depends on timing: the result is bit-identical across
+// runs, graph replays and data-parallel ranks.
+constexpr int kNormThreads = 256, kNormVecs = 8;
+constexpr long long kNormChunk = static_cast<long long>(kNormThreads) * 8 * kNormVecs;
+
+__device__ __forceinline__ double warp_sum_f64(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+// fixed-order CTA sum of one double per thread (every thread gets the result)
+__device__ __forceinline__ double block_sum_f64(double v, double* sh) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  v = warp_sum_f64(v);
+  __syncthreads();
+  if (lane == 0) sh[w] = v;
+  __syncthreads();
+  return warp_sum_f64(lane < (kNormThreads >> 5) ? sh[lane] : 0.0);
+}
+
+// transformers.optimization lambdas, in fp64 as the Python LambdaLR computes them
+__device__ double sched_lambda(int schedule, long long s, long long warmup, long long total) {
+  if (schedule == MM_SCHED_CONSTANT) return 1.0;
+  if (s < warmup) return static_cast<double>(s) / static_cast<double>(warmup > 1 ? warmup : 1);
+  if (schedule == MM_SCHED_CONSTANT_WITH_WARMUP) return 1.0;
+  const long long span = total - warmup > 1 ? total - warmup : 1;
+  if (schedule == MM_SCHED_LINEAR) return fmax(0.0, static_cast<double>(total - s) / static_cast<double>(span));
+  const double progress = static_cast<double>(s - warmup) / static_cast<double>(span);
+  return fmax(0.0, 0.5 * (1.0 + cospi(0.5 * 2.0 * progress)));  // cos(pi * 2 * num_cycles * progress)
+}
+
+__global__ void __launch_bounds__(kNormThreads) grad_norm_kernel(const long long* __restrict__ table, int n_tensors,
+                                                                 double* __restrict__ partials, mm_opt_state* st,
+                                                                 float max_norm, int skip_nonfinite, float base_lr,
+                                                                 int schedule, int warmup, int total) {
+  __shared__ double sh[32];
+  __shared__ bool last;
+  const int G = gridDim.x, tid = threadIdx.x;
+  const long long b = blockIdx.x;
+  double acc = 0.0;
+  long long base = 0;  // index of the current tensor's first chunk
+  for (int t = 0; t < n_tensors; ++t) {
+    const bf16* x = reinterpret_cast<const bf16*>(table[2 * t]);
+    const long long n = table[2 * t + 1];
+    const long long nc = (n + kNormChunk - 1) / kNormChunk;
+    const bool vec = (reinterpret_cast<uintptr_t>(x) & 15) == 0;
+    for (long long c = base + ((b - base % G) % G + G) % G; c < base + nc; c += G) {
+      const long long e0 = (c - base) * kNormChunk;
+      const long long e1 = e0 + kNormChunk < n ? e0 + kNormChunk : n;
+      float run = 0.f;
+      if (vec && e1 - e0 == kNormChunk) {
+        uint4 u[kNormVecs];
+#pragma unroll
+        for (int j = 0; j < kNormVecs; ++j)
+          u[j] = __ldg(reinterpret_cast<const uint4*>(x + e0) + j * kNormThreads + tid);
+#pragma unroll
+        for (int j = 0; j < kNormVecs; ++j) {
+          float f[8];
+          unpack8f(u[j], f);
+#pragma unroll
+          for (int k = 0; k < 8; ++k) run = fmaf(f[k], f[k], run);
+        }
+      } else {  // the last chunk of a tensor, or an unaligned tensor: scalar loads
+        for (long long i = e0 + tid; i < e1; i += kNormThreads) {
+          const float f = __bfloat162float(x[i]);
+          run = fmaf(f, f, run);
+        }
+      }
+      acc += static_cast<double>(run);
+    }
+    base += nc;
+  }
+  acc = block_sum_f64(acc, sh);
+  if (tid == 0) {
+    partials[blockIdx.x] = acc;
+    __threadfence();
+    last = atomicAdd(&st->arrived, 1) == G - 1;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  double tot = 0.0;
+  for (int i = tid; i < G; i += kNormThreads) tot += __ldcg(partials + i);
+  tot = block_sum_f64(tot, sh);
+  if (tid != 0) return;
+  st->arrived = 0;
+  const float norm = static_cast<float>(sqrt(tot));
+  const bool finite = isfinite(tot);
+  // torch.nn.utils.clip_grad_norm_: clamp(max_norm / (norm + 1e-6), max=1) in the norm's fp32 (NaN propagates)
+  float coef = 1.f;
+  if (max_norm > 0.f) {
+    coef = max_norm / (norm + 1e-6f);
+    coef = coef > 1.f ? 1.f : coef;
+  }
+  st->grad_norm = norm;
+  st->finite = finite ? 1 : 0;
+  st->clip_coef = coef;
+  if (finite || !skip_nonfinite) {
+    const int s = st->step;  // optimizer step s + 1 runs at lambda(s)
+    st->step = s + 1;
+    st->lr = static_cast<float>(static_cast<double>(base_lr) * sched_lambda(schedule, s, warmup, total));
+    st->apply = 1;
+  } else {
+    st->skipped += 1;
+    st->apply = 0;
   }
 }
 
@@ -821,6 +952,23 @@ extern "C" int32_t mm_colsum(const void* x, int64_t ldx, int32_t rows, int32_t c
   return check_launch("mm_colsum");
 }
 
+template <bool kSched>
+static void launch_adamw(void* p, const void* g, float* master, float* m, float* v, long long n, float lr, float beta1,
+                         float beta2, float eps, float weight_decay, float inv_bc1, float inv_bc2, float grad_scale,
+                         const int32_t* step_dev, const mm_opt_state* st, void* stream) {
+  const long long n8 = (AL16(p) && AL16(g) && AL16(master) && AL16(m) && AL16(v)) ? n / 8 : 0;
+  if (n8 > 0)
+    adamw_vec8_kernel<kSched><<<grid_for(n8, 256, 32), 256, 0, ST(stream)>>>((bf16*)p, (const bf16*)g, master, m, v, n8, lr,
+                                                                             beta1, beta2, eps, weight_decay, inv_bc1, inv_bc2,
+                                                                             grad_scale, step_dev, st);
+  if (n - 8 * n8 > 0) {  // unaligned tensors / the last n % 8 elements
+    const long long o = 8 * n8;
+    adamw_kernel<kSched><<<grid_for(n - o, 256), 256, 0, ST(stream)>>>((bf16*)p + o, (const bf16*)g + o, master + o, m + o,
+                                                                       v + o, n - o, lr, beta1, beta2, eps, weight_decay,
+                                                                       inv_bc1, inv_bc2, grad_scale, step_dev, st);
+  }
+}
+
 extern "C" int32_t mm_adamw(void* p, const void* g, float* master, float* m, float* v, int64_t n, float lr, float beta1,
                             float beta2, float eps, float weight_decay, int32_t step, const int32_t* step_dev,
                             float grad_scale, void* stream) {
@@ -828,18 +976,30 @@ extern "C" int32_t mm_adamw(void* p, const void* g, float* master, float* m, flo
   if (step <= 0) step = 1;
   const float inv_bc1 = 1.f / (1.f - powf(beta1, static_cast<float>(step)));
   const float inv_bc2 = 1.f / (1.f - powf(beta2, static_cast<float>(step)));
-  const long long n8 = (AL16(p) && AL16(g) && AL16(master) && AL16(m) && AL16(v)) ? n / 8 : 0;
-  if (n8 > 0)
-    adamw_vec8_kernel<<<grid_for(n8, 256, 32), 256, 0, ST(stream)>>>((bf16*)p, (const bf16*)g, master, m, v, n8, lr, beta1,
-                                                                     beta2, eps, weight_decay, inv_bc1, inv_bc2, grad_scale,
-                                                                     step_dev);
-  if (n - 8 * n8 > 0) {  // unaligned tensors / the last n % 8 elements
-    const long long o = 8 * n8;
-    adamw_kernel<<<grid_for(n - o, 256), 256, 0, ST(stream)>>>((bf16*)p + o, (const bf16*)g + o, master + o, m + o, v + o, n - o,
-                                                               lr, beta1, beta2, eps, weight_decay, inv_bc1, inv_bc2, grad_scale,
-                                                               step_dev);
-  }
+  launch_adamw<false>(p, g, master, m, v, n, lr, beta1, beta2, eps, weight_decay, inv_bc1, inv_bc2, grad_scale, step_dev,
+                      nullptr, stream);
   return check_launch("mm_adamw");
+}
+
+extern "C" int32_t mm_adamw_sched(void* p, const void* g, float* master, float* m, float* v, int64_t n, float beta1,
+                                  float beta2, float eps, float weight_decay, const mm_opt_state* state, void* stream) {
+  MM_REQUIRE(p && g && master && m && v && n > 0 && state, "mm_adamw_sched: bad arguments");
+  launch_adamw<true>(p, g, master, m, v, n, 0.f, beta1, beta2, eps, weight_decay, 1.f, 1.f, 1.f, nullptr, state, stream);
+  return check_launch("mm_adamw_sched");
+}
+
+extern "C" int32_t mm_grad_norm(const int64_t* table, int32_t n_tensors, double* partials, mm_opt_state* state,
+                                float max_norm, int32_t skip_nonfinite, float base_lr, int32_t schedule, int32_t warmup_steps,
+                                int32_t total_steps, void* stream) {
+  MM_REQUIRE(state && partials && n_tensors >= 0 && (n_tensors == 0 || table), "mm_grad_norm: bad arguments");
+  MM_REQUIRE(schedule >= MM_SCHED_CONSTANT && schedule <= MM_SCHED_COSINE && warmup_steps >= 0 && total_steps >= 0,
+             "mm_grad_norm: bad schedule");
+  // the grid is a constant (not a function of the device): the partition, hence every bit of the sum, is the same on
+  // every rank.  Without tensors the launch is the finisher alone.
+  const int grid = n_tensors > 0 ? MM_GRAD_NORM_PARTS : 1;
+  grad_norm_kernel<<<grid, kNormThreads, 0, ST(stream)>>>((const long long*)table, n_tensors, partials, state, max_norm,
+                                                          skip_nonfinite, base_lr, schedule, warmup_steps, total_steps);
+  return check_launch("mm_grad_norm");
 }
 
 extern "C" int32_t mm_align_softmax_bwd(const float* G, int64_t ldg, const void* Pp, int64_t ldp, const float* inv_l,

@@ -788,6 +788,57 @@ def adamw(p: torch.Tensor, g: torch.Tensor, master: torch.Tensor, m: torch.Tenso
                                 _ptr(step_dev), float(grad_scale), _stream()), "mm_adamw")
 
 
+# mm_opt_state (include/macaw_b200.h) as 8 int32 words; float fields are read through .view(torch.float32)
+OPT_STEP, OPT_SKIPPED, OPT_LR, OPT_CLIP_COEF, OPT_GRAD_NORM, OPT_FINITE, OPT_APPLY, OPT_ARRIVED = range(8)
+SCHEDULES = {"constant": 0, "constant_with_warmup": 1, "linear": 2, "cosine": 3}
+GRAD_NORM_PARTS = 1024  # MM_GRAD_NORM_PARTS
+
+
+def opt_state(device) -> torch.Tensor:
+    """A fresh mm_opt_state: step 0, nothing skipped, clip_coef 1, finite."""
+    st = torch.zeros((8,), dtype=torch.int32)
+    st.view(torch.float32)[OPT_CLIP_COEF] = 1.0
+    st[OPT_FINITE] = 1
+    return st.to(device)
+
+
+def grad_table(grads) -> torch.Tensor:
+    """Device int64 (n, 2) table of (address, numel) of contiguous bf16 gradients (the input of grad_norm)."""
+    rows = []
+    for g in grads:
+        _cuda(g, _BF16, "gradient")
+        if not g.is_contiguous():
+            raise RuntimeError("macaw_b200: grad_norm needs contiguous gradients")
+        rows.append((g.data_ptr(), g.numel()))
+    return torch.tensor(rows, dtype=torch.int64).reshape(-1, 2).to(torch.cuda.current_device())
+
+
+def grad_norm(table: Optional[torch.Tensor], state: torch.Tensor, partials: torch.Tensor, *, max_norm: float = 0.0,
+              skip_nonfinite: bool = False, base_lr: float = 0.0, schedule: str = "constant", warmup_steps: int = 0,
+              total_steps: int = 0) -> None:
+    """mm_grad_norm: global L2 norm of the gradients in `table` (None / empty: no pass) into the optimizer state, then the
+    step's clip coefficient, step count and learning rate (see include/macaw_b200.h)."""
+    _cuda(state, torch.int32, "state"); _cuda(partials, torch.float64, "partials")
+    assert state.numel() == 8 and partials.numel() >= GRAD_NORM_PARTS
+    n = 0 if table is None else table.shape[0]
+    if n:
+        _cuda(table, torch.int64, "table")
+        assert table.is_contiguous() and table.shape[1] == 2
+    _check(_lib.load().mm_grad_norm(_ptr(table) if n else None, n, partials.data_ptr(), state.data_ptr(), float(max_norm),
+                                    int(bool(skip_nonfinite)), float(base_lr), SCHEDULES[schedule], int(warmup_steps),
+                                    int(total_steps), _stream()), "mm_grad_norm")
+
+
+def adamw_sched(p: torch.Tensor, g: torch.Tensor, master: torch.Tensor, m: torch.Tensor, v: torch.Tensor, *, beta1: float,
+                beta2: float, eps: float, weight_decay: float, state: torch.Tensor) -> None:
+    """mm_adamw_sched: AdamW with lr, gradient multiplier, step and skip flag read from the device optimizer state."""
+    _cuda(p, ACT(), "p"); _cuda(g, ACT(), "g"); _cuda(state, torch.int32, "state")
+    assert p.is_contiguous() and g.is_contiguous() and master.numel() == p.numel() and g.numel() == p.numel()
+    _check(_lib.load().mm_adamw_sched(p.data_ptr(), g.data_ptr(), master.data_ptr(), m.data_ptr(), v.data_ptr(), p.numel(),
+                                      float(beta1), float(beta2), float(eps), float(weight_decay), state.data_ptr(),
+                                      _stream()), "mm_adamw_sched")
+
+
 def cast_bf16(x: torch.Tensor) -> torch.Tensor:
     """fp16 contiguous tensor -> bf16 copy (mm_cast_f16_bf16): the alignment backward runs in bf16 (gradient range)."""
     _cuda(x, _F16, "x")
